@@ -4,6 +4,7 @@ data-parallel TorchJob at N worker-replica GPUs, with the allreduce's achieved b
 the NVLink roofline, next to the reference-style gloo/CPU torchjob on the box's host cores.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference|nccl]
+                  [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
       --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -198,6 +199,26 @@ def parity_check(rep, sizes, world, zero_copy, stream):
                        "bit for bit on every replica before timing"}
 
 
+DUMP_SAMPLE = 1 << 22   # elements kept of each flattened array: 16 MiB per file as float32
+
+
+def dump_outputs(out_dir, model, loss):
+    """What the caller of the last timed step holds afterwards, as float32 .npy files: its loss, the
+    averaged gradients (the bucket exchange's output) and the updated parameters.  The two flattened
+    arrays of 25.6 M elements are cut to the same fixed, seeded sample of DUMP_SAMPLE elements."""
+    import numpy as np
+    import torch
+    params = list(model.parameters())
+    flat = {"grads": torch.cat([p.grad.detach().flatten().float() for p in params]),
+            "params": torch.cat([p.detach().flatten().float() for p in params])}
+    n = flat["params"].numel()
+    idx = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:DUMP_SAMPLE].sort().values
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "loss.npy"), np.array([loss], dtype=np.float32))
+    for name, t in flat.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t[idx.to(t.device)].cpu().numpy())
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -227,7 +248,11 @@ def run_ours(args):
 
     rep = init_replica(device=local)
     dev = rep.device
-    torch.backends.cudnn.benchmark = True
+    # Dumped outputs are compared between runs and builds, so a dumping run takes cuDNN's
+    # deterministic algorithms instead of each run's fastest: tens of bf16 training steps amplify
+    # one step's last-bit differences until the weights no longer agree.
+    torch.backends.cudnn.benchmark = not args.dump_outputs
+    torch.backends.cudnn.deterministic = bool(args.dump_outputs)
     B = args.batch
     nccl_only = args.impl == "nccl"
 
@@ -374,10 +399,13 @@ def run_ours(args):
 
     for i in range(2):
         e2e_step(i)
-    ms_e2e = timed(e2e_step, args.steps)
+    last = {}
+    ms_e2e = timed(lambda i: last.__setitem__("loss", e2e_step(i)), args.steps)
     clocks = sampler.stop() if rank == 0 else None
     hook.drain_events()
     rep.comm.status()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, ddp, last["loss"])
 
     # ---- roofline of the dominant kernel of OUR path (the bucket exchange) -----------------------
     # CUDA events on the comm stream around the exchange kernel alone; the 1-warp arrival in front of
@@ -537,6 +565,9 @@ def run_ours(args):
                                "hot-path kernel runs and is measured in-step (gpu_launches counts "
                                "those launches), as the reference's own hook does (div_(1) + "
                                "allreduce)")
+    if args.dump_outputs:
+        line["dump_outputs"] = {"dir": args.dump_outputs,
+                                "cudnn": "deterministic algorithms, benchmark mode off"}
     if nccl is not None:
         line["nccl"] = nccl
         line["vs_nccl"] = {"step": value / nccl["value"], "e2e": e2e_value / nccl["e2e"]["value"],
@@ -571,7 +602,12 @@ def main():
     ap.add_argument("--no-nccl", action="store_true", help="skip the stock DDP+NCCL comparison leg")
     ap.add_argument("--cpu-steps", type=int, default=3)
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed as "
+                         "DIR/<name>.npy (the run uses cuDNN's deterministic algorithms)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.impl == "reference":
         return run_reference(args)
     return run_ours(args)

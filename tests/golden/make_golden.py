@@ -11,7 +11,8 @@ Fixtures
       native-dtype bf16 all_reduce of bf16(x)/N ["bf16_native"] (informational: gloo sums in bf16).
   sampler.json                    DistributedSampler indices for several (len, world, epoch, seed).
   mlp_torchjob_n2/                BASELINE config 0: 2-layer MLP, 1 master + 1 worker, gloo: losses,
-      per-bucket pre/post tensors, argmax, final weights of rank 0 and 1.
+      per-bucket pre/post tensors, argmax, final weights of rank 0 and 1 (the flat arrays as a
+      seeded sample of their elements, indices in "sample_index").
 """
 from __future__ import annotations
 
@@ -30,6 +31,7 @@ sys.path.insert(0, os.path.join(ROOT, "tests"))
 
 COUNT = 4099
 SEED = 4242
+MLP_SAMPLE = 1 << 12
 
 
 def _rank(rank, world, port, q):
@@ -127,12 +129,32 @@ def make_sampler():
         json.dump(out, f)
 
 
+def shrink_mlp_dump(d):
+    """Keep the same fixed, seeded sample of MLP_SAMPLE elements of every flat per-parameter array
+    (bucket tensors, final weights) so that each rank's fixture stays under 1 MB; the allreduce is
+    element-wise, so the sampled elements are checked exactly as the full buckets would be."""
+    for name in sorted(os.listdir(d)):
+        if not name.endswith(".npz"):
+            continue
+        path = os.path.join(d, name)
+        with np.load(path) as z:
+            arrays = {k: z[k] for k in z.files}
+        n = arrays["final_flat"].size
+        idx = np.sort(np.random.RandomState(SEED).choice(n, MLP_SAMPLE, replace=False))
+        for k, a in arrays.items():
+            if a.shape == (n,):
+                arrays[k] = a[idx]
+        arrays["sample_index"] = idx.astype(np.int32)
+        np.savez_compressed(path, **arrays)
+
+
 def make_mlp():
     from oracle import gloo_torchjob
     d = os.path.join(HERE, "mlp_torchjob_n2")
     shutil.rmtree(d, ignore_errors=True)
     res = gloo_torchjob.run("mlp", world=2, steps=2, warmup=0, batch=64, threads=1, dtype="f32",
                             dump=d, job="golden-mlp")
+    shrink_mlp_dump(d)
     with open(os.path.join(d, "run.json"), "w") as f:
         json.dump(dict(losses=res["losses"], steps=2, batch=64, lr=0.01, world=2), f)
 

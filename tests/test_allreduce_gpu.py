@@ -186,6 +186,41 @@ def test_golden_gloo_vectors(tok_lib, n_gpus):
         assert s["bad"] == 0 and s["total"] == len(cases) * world, s
 
 
+def test_long_rendezvous_path(tok_lib, tmp_path):
+    """A rendezvous path longer than a Unix socket address holds (108 bytes, easily reached under a
+    deep temporary or shared directory) still forms the group and exchanges buckets."""
+    import threading
+    import torch
+    from torch_on_k8s_b200.comm import Communicator
+    os.environ.update(SHARED_ENV)
+    d = tmp_path / ("d" * 120)
+    d.mkdir()
+    path = str(d / "r")
+    outs, errs = {}, []
+
+    def body(r):
+        try:
+            torch.cuda.set_device(0)
+            comm = Communicator("long", r, 2, 0, rendezvous_path=path)
+            st = torch.cuda.Stream(device=0)
+            with torch.cuda.stream(st):
+                x = torch.full((4096,), float(r + 1), device="cuda:0")
+                comm.allreduce_bucket(x, x, scale=0.5, stream=st)
+                st.synchronize()
+            comm.status()
+            outs[r] = x.cpu()
+            comm.close()
+        except Exception as e:  # noqa: BLE001
+            errs.append(repr(e))
+
+    ts = [threading.Thread(target=body, args=(r,)) for r in range(2)]
+    [t.start() for t in ts]
+    [t.join(120) for t in ts]
+    assert not errs, errs
+    for r in range(2):
+        assert torch.equal(outs[r], torch.full((4096,), 1.5)), r
+
+
 @pytest.mark.parametrize("world", [2, 3, 4])
 def test_zero_copy_symmetric_pool(tok_lib, n_gpus, world):
     """Buckets allocated in the symmetric pool (torch.cuda.MemPool over tok_pool_malloc) are

@@ -114,8 +114,15 @@ def test_permanent_exit_code_fails_job(tok_lib, tmp_path, monkeypatch):
     monkeypatch.setenv("FAIL_CODE", "1")      # permanent under ExitCode (failover.go:64-76)
     ctl = Controller(num_gpus=2)
     uid = ctl.submit(manifest("pf", free_port()))
-    res = ctl.run_until_done(timeout=120)
-    assert res[uid] == "Failed"
+    try:
+        res = ctl.run_until_done(timeout=120)
+        assert res[uid] == "Failed"
+    finally:
+        # cleanPodPolicy None keeps the worker, which would wait out gloo's 30-minute rendezvous
+        # timeout for the failed master: stop it so that the test leaves no process behind
+        for reps in ctl.jobs[uid].replicas.values():
+            for r in reps.values():
+                ctl._kill(r)
 
 
 def test_replica_sampler_matches_distributed_sampler_goldens():

@@ -95,7 +95,7 @@ def test_sampler_sharding_golden():
 def test_mlp_bucket_golden():
     """BASELINE config 0 (MLP, 1 master + 1 worker, gloo): every recorded gradient bucket's
     post-allreduce tensor equals the oracle applied to the two replicas' pre tensors, bit for bit
-    (N=2, fp32)."""
+    (N=2, fp32), on the fixture's seeded sample of bucket elements."""
     d = os.path.join(GOLD, "mlp_torchjob_n2")
     r0 = np.load(os.path.join(d, "rank0.npz"))
     r1 = np.load(os.path.join(d, "rank1.npz"))

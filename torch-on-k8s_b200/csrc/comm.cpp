@@ -527,10 +527,31 @@ int exchange(tok_comm* c) {
   struct sockaddr_un addr;
   memset(&addr, 0, sizeof(addr));
   addr.sun_family = AF_UNIX;
-  if (star.path.size() >= sizeof(addr.sun_path))
-    return fail(TOK_ERR_INVALID, "rendezvous path too long (%zu >= %zu): %s", star.path.size(),
+  // sun_path holds 107 characters.  A longer path names the same socket file through this
+  // process's descriptor of its directory, /proc/self/fd/<dir>/<name>, which every replica opens
+  // for itself; the directory descriptor only has to live until bind() / connect().
+  std::string sock = star.path;
+  struct DirFd {
+    int fd = -1;
+    ~DirFd() {
+      if (fd >= 0) close(fd);
+    }
+  } dir;
+  if (sock.size() >= sizeof(addr.sun_path)) {
+    const size_t slash = star.path.rfind('/');
+    const std::string parent =
+        slash == std::string::npos ? "." : (slash == 0 ? "/" : star.path.substr(0, slash));
+    dir.fd = open(parent.c_str(), O_PATH | O_DIRECTORY | O_CLOEXEC);
+    if (dir.fd < 0)
+      return fail(TOK_ERR_RENDEZVOUS, "rendezvous directory %s: %s", parent.c_str(),
+                  strerror(errno));
+    sock = "/proc/self/fd/" + std::to_string(dir.fd) + "/" +
+           star.path.substr(slash == std::string::npos ? 0 : slash + 1);
+  }
+  if (sock.size() >= sizeof(addr.sun_path))
+    return fail(TOK_ERR_INVALID, "rendezvous file name too long (%zu >= %zu): %s", sock.size(),
                 sizeof(addr.sun_path), star.path.c_str());
-  strcpy(addr.sun_path, star.path.c_str());
+  strcpy(addr.sun_path, sock.c_str());
 
   Hello me;
   memset(&me, 0, sizeof(me));
