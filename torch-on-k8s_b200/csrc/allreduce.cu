@@ -65,6 +65,9 @@ __device__ __forceinline__ unsigned long long ld_relaxed_sys(const unsigned long
   asm volatile("ld.relaxed.sys.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
   return v;
 }
+__device__ __forceinline__ void st_relaxed_sys(uint32_t* p, uint32_t v) {
+  asm volatile("st.relaxed.sys.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
+}
 __device__ __forceinline__ void st_relaxed_sys(unsigned long long* p, unsigned long long v) {
   asm volatile("st.relaxed.sys.global.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory");
 }
@@ -73,6 +76,9 @@ __device__ __forceinline__ void fence_sys() { asm volatile("fence.acq_rel.sys;" 
 // to the multicast object (release: ordered after this CTA's data writes, cumulative over bar.sync).
 __device__ __forceinline__ void multimem_red_release_add(uint32_t* mc_ptr, uint32_t v) {
   asm volatile("multimem.red.release.sys.global.add.u32 [%0], %1;" ::"l"(mc_ptr), "r"(v) : "memory");
+}
+__device__ __forceinline__ void multimem_red_relaxed_add(uint32_t* mc_ptr, uint32_t v) {
+  asm volatile("multimem.red.relaxed.sys.global.add.u32 [%0], %1;" ::"l"(mc_ptr), "r"(v) : "memory");
 }
 // Data written by other GPUs during this kernel is always read at system scope (served by the
 // home L2, never by a stale local L1 line).
@@ -303,43 +309,45 @@ __device__ __forceinline__ int warp_spin(const KArgs& a, const uint32_t* word, u
   }
 }
 
-// ACQUIRE: fence (system scope) after the wait.  Needed when the CTA goes on to read what the peers
-// wrote; the trailing barrier of the zero-copy kernels is followed by nothing but the kernel's end
-// (the next kernel starts with a clean L1 and reads local memory through the coherent L2), so it
-// skips the fence — measured (tools/barrier_bench.py, 8 GPUs, 64 CTAs): signalling alone 2.0 us,
-// with release + acquire fences 10.5 us; the fences, not the flags, are what a barrier costs.
-template <bool ACQUIRE = true>
-__device__ __forceinline__ bool cta_barrier(const KArgs& a, uint32_t target, int* s_fail) {
-  __syncthreads();
-  if (threadIdx.x < 32) {
-    const int lane = threadIdx.x;
-    const uint32_t* word;
-    uint32_t want;
-    bool polls;
-    if (a.mc != nullptr) {
-      if (lane == 0)
-        multimem_red_release_add(reinterpret_cast<uint32_t*>(a.mc + kMcntOff) + blockIdx.x, 1u);
-      word = reinterpret_cast<const uint32_t*>(a.peer[a.rank] + kMcntOff) + blockIdx.x;
-      want = target * static_cast<uint32_t>(a.world);
-      polls = lane == 0;
-    } else {
-      polls = lane < a.world;
-      if (polls)
-        st_release_sys(reinterpret_cast<uint32_t*>(a.peer[lane]) + (blockIdx.x * kMaxWorld + a.rank),
-                       target);
-      word = reinterpret_cast<const uint32_t*>(a.peer[a.rank]) +
-             (blockIdx.x * kMaxWorld + (polls ? lane : 0));
-      want = target;
+// Warp 0's part of the barrier on flag slot `slot`: signal `target` through the multicast counter
+// (mc) or the P2P flags, as a release or a relaxed store, wait for every replica, record a failure
+// in *s_fail, and fence if `acquire`.  The exchange kernels signal with release; relaxed signalling
+// only exists so that tools/barrier_bench.py can time the flags without the ordering.
+__device__ __forceinline__ void warp_barrier(const KArgs& a, uint32_t slot, uint32_t target, bool mc,
+                                             bool release, bool acquire, int* s_fail) {
+  const int lane = threadIdx.x;
+  const uint32_t* word;
+  uint32_t want;
+  bool polls;
+  if (mc) {
+    uint32_t* cnt = reinterpret_cast<uint32_t*>(a.mc + kMcntOff) + slot;
+    if (lane == 0) {
+      if (release)
+        multimem_red_release_add(cnt, 1u);
+      else
+        multimem_red_relaxed_add(cnt, 1u);
     }
-    const int code = warp_spin(a, word, want, polls, 2u);
-    if (code != 0 && lane == 0) {
-      a.hostctl[kCtlStatus] = code;
-      *s_fail = 1;
+    word = reinterpret_cast<const uint32_t*>(a.peer[a.rank] + kMcntOff) + slot;
+    want = target * static_cast<uint32_t>(a.world);
+    polls = lane == 0;
+  } else {
+    polls = lane < a.world;
+    if (polls) {
+      uint32_t* flag = reinterpret_cast<uint32_t*>(a.peer[lane]) + (slot * kMaxWorld + a.rank);
+      if (release)
+        st_release_sys(flag, target);
+      else
+        st_relaxed_sys(flag, target);
     }
-    if (ACQUIRE) fence_sys();  // acquire side of the flag hand-off; bar.sync extends it to the CTA
+    word = reinterpret_cast<const uint32_t*>(a.peer[a.rank]) + (slot * kMaxWorld + (polls ? lane : 0));
+    want = target;
   }
-  __syncthreads();
-  return *s_fail == 0;
+  const int code = warp_spin(a, word, want, polls, 2u);
+  if (code != 0 && lane == 0) {
+    a.hostctl[kCtlStatus] = code;
+    *s_fail = 1;
+  }
+  if (acquire) fence_sys();  // acquire side of the flag hand-off; bar.sync extends it to the CTA
 }
 
 // Optional phase timestamps for tools/phase_breakdown.py (never enabled on the product path).
@@ -351,21 +359,44 @@ struct CtaState {
   uint32_t seq;      // launches completed before this one (buffer parity)
   uint32_t bar;      // barriers this CTA index has passed
   uint32_t arrived;  // verdict of the last arrive_kernel (0 = every replica's bucket is ready)
+  int* fail;         // CtaShared::fail
 };
 
-__device__ __forceinline__ CtaState cta_begin(const KArgs& a, uint32_t* s_words, int* s_fail) {
+// Declared __shared__ by each kernel, not here: a kernel's own variable lets the compiler drop the
+// words that kernel never reads.
+struct CtaShared {
+  uint32_t words[3];  // CtaState's first three fields, read once by thread 0
+  int fail;           // set by a barrier that was given up
+};
+
+__device__ __forceinline__ CtaState cta_begin(const KArgs& a, CtaShared& sh) {
   if (threadIdx.x == 0) {
-    s_words[0] = a.ctr[kCtrCallSeq];
-    s_words[1] = a.ctr[blockIdx.x];
-    s_words[2] = a.ctr[kCtrArriveCode];
-    *s_fail = 0;
+    sh.words[0] = a.ctr[kCtrCallSeq];
+    sh.words[1] = a.ctr[blockIdx.x];
+    sh.words[2] = a.ctr[kCtrArriveCode];
+    sh.fail = 0;
   }
   __syncthreads();
   CtaState st;
-  st.seq = s_words[0];
-  st.bar = s_words[1];
-  st.arrived = s_words[2];
+  st.seq = sh.words[0];
+  st.bar = sh.words[1];
+  st.arrived = sh.words[2];
+  st.fail = &sh.fail;
   return st;
+}
+
+// ACQUIRE: fence (system scope) after the wait.  Needed when the CTA goes on to read what the peers
+// wrote; the trailing barrier of the zero-copy kernels is followed by nothing but the kernel's end
+// (the next kernel starts with a clean L1 and reads local memory through the coherent L2), so it
+// skips the fence — measured (tools/barrier_bench.py, 8 GPUs, 64 CTAs): signalling alone 2.0 us,
+// with release + acquire fences 10.5 us; the fences, not the flags, are what a barrier costs.
+template <bool ACQUIRE = true>
+__device__ __forceinline__ bool cta_barrier(const KArgs& a, CtaState& st) {
+  st.bar += 1;
+  __syncthreads();
+  if (threadIdx.x < 32) warp_barrier(a, blockIdx.x, st.bar, a.mc != nullptr, true, ACQUIRE, st.fail);
+  __syncthreads();
+  return *st.fail == 0;
 }
 
 // Last CTA out bumps the launch sequence (selects the other staging buffer next time); works under
@@ -381,6 +412,56 @@ __device__ __forceinline__ void cta_end(const KArgs& a, const CtaState& st) {
       a.ctr[kCtrCallSeq] = st.seq + 1;
     }
   }
+}
+
+template <class T>
+__device__ __forceinline__ T min_sz(T a, T b) {
+  return a < b ? a : b;
+}
+
+struct Range {
+  size_t lo, hi;
+};
+
+// The PRE/POST scale pair and a CTA's slab: CTA b owns packs [b * packs_per_cta, +packs_per_cta),
+// clipped to `end`.
+struct Slab {
+  float pre;   // each contribution's scale: scale (PRE) or 1 (POST)
+  float post;  // the sum's scale: 1 (PRE) or scale (POST)
+  size_t lo, hi;
+  size_t M;  // sub-slab length
+  // The sub-slab replica `rank` reduces (two-shot, NVLS): M packs from lo + rank * M, clipped to
+  // the slab.  Call it where it is used; computed up front, it is scheduled ahead of the barrier.
+  __device__ __forceinline__ Range sub(int rank) const {
+    const size_t slo = min_sz(lo + static_cast<size_t>(rank) * M, hi);
+    return Range{slo, min_sz(slo + M, hi)};
+  }
+};
+
+__device__ __forceinline__ Slab cta_slab(const KArgs& a, size_t end) {
+  Slab s;
+  s.pre = (a.flags & TOK_FLAG_SCALE_POST) ? 1.f : a.scale;
+  s.post = (a.flags & TOK_FLAG_SCALE_POST) ? a.scale : 1.f;
+  s.lo = static_cast<size_t>(blockIdx.x) * a.packs_per_cta;
+  s.hi = min_sz(s.lo + a.packs_per_cta, end);
+  s.M = a.packs_per_cta / a.world;
+  return s;
+}
+
+// The streaming loop over packs [lo, hi): each thread issues U independent loads, kThreads packs
+// apart, before the first of their U stores, then finishes one pack at a time.  Each caller's U was
+// tuned for its load.
+template <int U, class Load, class Store>
+__device__ __forceinline__ void stream(size_t lo, size_t hi, Load load, Store store) {
+  size_t i = lo + threadIdx.x;
+  for (; i + (U - 1) * kThreads < hi; i += U * kThreads) {
+    decltype(load(i)) r[U];
+#pragma unroll
+    for (int u = 0; u < U; ++u) r[u] = load(i + u * kThreads);
+#pragma unroll
+    for (int u = 0; u < U; ++u) store(i + u * kThreads, r[u]);
+  }
+  for (; i < hi; i += kThreads) store(i, load(i));
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -418,6 +499,17 @@ struct AR {
     }
     return CW::from_f32(v);
   }
+  // wire pack * post (the sum's scale), through fp32
+  static __device__ __forceinline__ RW scale_wire(RW w, float post) {
+    if (post != 1.f) {
+      float v[P];
+      CW::to_f32(w, v);
+#pragma unroll
+      for (int k = 0; k < P; ++k) v[k] *= post;
+      w = CW::from_f32(v);
+    }
+    return w;
+  }
   // wire pack -> out (vector store, or guarded scalar stores for the partial last pack)
   static __device__ __forceinline__ void wire_to_out(const KArgs& a, size_t pack, const RW& w) {
     OUT* out = static_cast<OUT*>(a.out);
@@ -447,16 +539,8 @@ struct AR {
     const RI* in = static_cast<const RI*>(a.in);
     const size_t full = a.count / P;
     const size_t hv = hi < full ? hi : full;
-    constexpr int U = 4;
-    size_t i = lo + threadIdx.x;
-    for (; i + (U - 1) * kThreads < hv; i += U * kThreads) {
-      RI r[U];
-#pragma unroll
-      for (int u = 0; u < U; ++u) r[u] = __ldcs(in + i + u * kThreads);
-#pragma unroll
-      for (int u = 0; u < U; ++u) dst[i + u * kThreads] = in_to_wire(r[u], pre);
-    }
-    for (; i < hv; i += kThreads) dst[i] = in_to_wire(__ldcs(in + i), pre);
+    stream<4>(lo, hv, [&](size_t i) { return __ldcs(in + i); },
+              [&](size_t i, const RI& r) { dst[i] = in_to_wire(r, pre); });
     if (threadIdx.x == 0 && full < a.total_packs && full >= lo && full < hi)
       dst[full] = in_tail_to_wire(a, full, pre);
   }
@@ -470,43 +554,25 @@ struct AR {
     for (int p = 0; p < kMaxWorld; ++p)
       dst[p] = reinterpret_cast<RW*>(a.peer[p < a.world ? p : 0] + a.stage_off[q] +
                                      static_cast<size_t>(a.rank) * a.slot_bytes);
-    const size_t full = a.count / P;
-    const size_t hv = hi < full ? hi : full;
-    constexpr int U = 2;
-    size_t i = lo + threadIdx.x;
-    for (; i + (U - 1) * kThreads < hv; i += U * kThreads) {
-      RI r[U];
-#pragma unroll
-      for (int u = 0; u < U; ++u) r[u] = __ldcs(in + i + u * kThreads);
-#pragma unroll
-      for (int u = 0; u < U; ++u) {
-        const RW w = in_to_wire(r[u], pre);
-#pragma unroll
-        for (int p = 0; p < kMaxWorld; ++p)
-          if (p < a.world) dst[p][i + u * kThreads] = w;
-      }
-    }
-    for (; i < hv; i += kThreads) {
-      const RW w = in_to_wire(__ldcs(in + i), pre);
+    auto put = [&](size_t i, const RW& w) {
 #pragma unroll
       for (int p = 0; p < kMaxWorld; ++p)
         if (p < a.world) dst[p][i] = w;
-    }
-    if (threadIdx.x == 0 && full < a.total_packs && full >= lo && full < hi) {
-      const RW w = in_tail_to_wire(a, full, pre);
-#pragma unroll
-      for (int p = 0; p < kMaxWorld; ++p)
-        if (p < a.world) dst[p][full] = w;
-    }
+    };
+    const size_t full = a.count / P;
+    const size_t hv = hi < full ? hi : full;
+    stream<2>(lo, hv, [&](size_t i) { return __ldcs(in + i); },
+              [&](size_t i, const RI& r) { put(i, in_to_wire(r, pre)); });
+    if (threadIdx.x == 0 && full < a.total_packs && full >= lo && full < hi)
+      put(full, in_tail_to_wire(a, full, pre));
   }
 
-  // ---- rank-ordered fp32 reduction of packs [lo, hi) from src[0..world) --------------------------
-  // Every load of a batch is issued before the first add: world x U 16-byte requests in flight per
-  // thread hide the ~2 us NVLink round trip.  `mine` (two-shot) receives the reduced wire pack in
-  // place so that peers can pull it in phase 2.
-  template <int MAXW, int U>
-  static __device__ __forceinline__ void reduce_packs(const KArgs& a, const RW* const (&src)[kMaxWorld],
-                                                      RW* mine, size_t lo, size_t hi, float post) {
+  // The streaming loop over rows: pack i of src[0..world).  All U x world loads of a batch are issued
+  // before the first row is reduced; world x U 16-byte requests in flight per thread hide the ~2 us
+  // NVLink round trip.
+  template <int MAXW, int U, class Row>
+  static __device__ __forceinline__ void stream_rows(const KArgs& a, const RW* const* src, size_t lo,
+                                                     size_t hi, Row row) {
     size_t i = lo + threadIdx.x;
     for (; i + (U - 1) * kThreads < hi; i += U * kThreads) {
       RW r[U][MAXW];
@@ -516,29 +582,23 @@ struct AR {
         for (int p = 0; p < MAXW; ++p)
           if (p < a.world) r[u][p] = ld_sys(src[p] + i + u * kThreads);
 #pragma unroll
-      for (int u = 0; u < U; ++u) {
-        float acc[P];
-        CW::to_f32(r[u][0], acc);
-#pragma unroll
-        for (int p = 1; p < MAXW; ++p)
-          if (p < a.world) {
-            float v[P];
-            CW::to_f32(r[u][p], v);
-#pragma unroll
-            for (int k = 0; k < P; ++k) acc[k] += v[k];
-          }
-#pragma unroll
-        for (int k = 0; k < P; ++k) acc[k] *= post;
-        const RW w = CW::from_f32(acc);
-        if (mine) mine[i + u * kThreads] = w;
-        wire_to_out(a, i + u * kThreads, w);
-      }
+      for (int u = 0; u < U; ++u) row(r[u], i + u * kThreads);
     }
     for (; i < hi; i += kThreads) {
       RW r[MAXW];
 #pragma unroll
       for (int p = 0; p < MAXW; ++p)
         if (p < a.world) r[p] = ld_sys(src[p] + i);
+      row(r, i);
+    }
+  }
+
+  // ---- rank-ordered fp32 reduction of packs [lo, hi) from src[0..world) --------------------------
+  // `mine` (two-shot) receives the reduced wire pack in place so that peers can pull it in phase 2.
+  template <int MAXW, int U>
+  static __device__ __forceinline__ void reduce_packs(const KArgs& a, const RW* const (&src)[kMaxWorld],
+                                                      RW* mine, size_t lo, size_t hi, float post) {
+    auto one = [&](const RW (&r)[MAXW], size_t idx) {
       float acc[P];
       CW::to_f32(r[0], acc);
 #pragma unroll
@@ -552,9 +612,10 @@ struct AR {
 #pragma unroll
       for (int k = 0; k < P; ++k) acc[k] *= post;
       const RW w = CW::from_f32(acc);
-      if (mine) mine[i] = w;
-      wire_to_out(a, i, w);
-    }
+      if (mine) mine[idx] = w;
+      wire_to_out(a, idx, w);
+    };
+    stream_rows<MAXW, U>(a, src, lo, hi, one);
   }
 
   static __device__ __forceinline__ void reduce_dispatch(const KArgs& a,
@@ -609,16 +670,8 @@ struct AR {
   // ---- phase 2 (NVLS): local staging -> out over packs [lo, hi) -----------------------------------
   static __device__ __forceinline__ void copy_out(const KArgs& a, const RW* src, size_t lo,
                                                   size_t hi) {
-    constexpr int U = 8;
-    size_t i = lo + threadIdx.x;
-    for (; i + (U - 1) * kThreads < hi; i += U * kThreads) {
-      RW r[U];
-#pragma unroll
-      for (int u = 0; u < U; ++u) r[u] = ld_sys(src + i + u * kThreads);
-#pragma unroll
-      for (int u = 0; u < U; ++u) wire_to_out(a, i + u * kThreads, r[u]);
-    }
-    for (; i < hi; i += kThreads) wire_to_out(a, i, ld_sys(src + i));
+    stream<8>(lo, hi, [&](size_t i) { return ld_sys(src + i); },
+              [&](size_t i, const RW& w) { wire_to_out(a, i, w); });
   }
 
   // ---- NVLS phase 1: in-switch reduce of my sub-slab, broadcast of the result ----------------------
@@ -627,25 +680,8 @@ struct AR {
                                                      size_t hi, float post) {
     using M = MM<WIRE, sizeof(RW)>;
     RW* mc = reinterpret_cast<RW*>(mc_stage);
-    auto finish = [&](size_t idx, RW r) {
-      if (post != 1.f) {
-        float v[P];
-        CW::to_f32(r, v);
-#pragma unroll
-        for (int k = 0; k < P; ++k) v[k] *= post;
-        r = CW::from_f32(v);
-      }
-      M::st(mc + idx, r);
-    };
-    size_t i = lo + threadIdx.x;
-    for (; i + (U - 1) * kThreads < hi; i += U * kThreads) {
-      RW r[U];
-#pragma unroll
-      for (int u = 0; u < U; ++u) r[u] = M::ld_reduce(mc + i + u * kThreads);
-#pragma unroll
-      for (int u = 0; u < U; ++u) finish(i + u * kThreads, r[u]);
-    }
-    for (; i < hi; i += kThreads) finish(i, M::ld_reduce(mc + i));
+    stream<U>(lo, hi, [&](size_t i) { return M::ld_reduce(mc + i); },
+              [&](size_t i, const RW& r) { M::st(mc + i, scale_wire(r, post)); });
   }
 
   // ---- zero-copy two-shot: reduce packs [lo, hi) straight from every replica's bucket (rank order,
@@ -682,24 +718,7 @@ struct AR {
       for (int p = 0; p < MAXW; ++p)
         if (p < a.world) buf[p][idx] = w;
     };
-    size_t i = lo + threadIdx.x;
-    for (; i + (U - 1) * kThreads < hi; i += U * kThreads) {
-      RW r[U][MAXW];
-#pragma unroll
-      for (int u = 0; u < U; ++u)
-#pragma unroll
-        for (int p = 0; p < MAXW; ++p)
-          if (p < a.world) r[u][p] = ld_sys(buf[p] + i + u * kThreads);
-#pragma unroll
-      for (int u = 0; u < U; ++u) one(r[u], i + u * kThreads);
-    }
-    for (; i < hi; i += kThreads) {
-      RW r[MAXW];
-#pragma unroll
-      for (int p = 0; p < MAXW; ++p)
-        if (p < a.world) r[p] = ld_sys(buf[p] + i);
-      one(r, i);
-    }
+    stream_rows<MAXW, U>(a, buf, lo, hi, one);
   }
 
   // A failed barrier leaves the bucket half exchanged: overwrite this CTA's slab of `out` with NaN so
@@ -711,12 +730,15 @@ struct AR {
     const OUT nan = CO::from_scalar(__int_as_float(0x7fc00000));
     for (size_t e = e_lo + threadIdx.x; e < e_hi; e += kThreads) out[e] = nan;
   }
-};
 
-template <class T>
-__device__ __forceinline__ T min_sz(T a, T b) {
-  return a < b ? a : b;
-}
+  // The end of an exchange CTA: poison on failure, last phase stamp, hand over the launch state.
+  static __device__ __forceinline__ void finish(const KArgs& a, const CtaState& st, const Slab& s,
+                                                bool ok) {
+    if (!ok) poison(a, s.lo, s.hi);
+    dbg_stamp(a, 5);
+    cta_end(a, st);
+  }
+};
 
 // world == 1: fused scale/cast only (HBM bound: S_in + S_out).  ONE even wave: CTA b owns the
 // contiguous packs [b*L, (b+1)*L) with L = packs_per_cta chosen by the host so that the grid is at
@@ -725,34 +747,16 @@ __device__ __forceinline__ T min_sz(T a, T b) {
 template <class IN, class WIRE, class OUT>
 __global__ void __launch_bounds__(kThreads, 2) local_kernel(const __grid_constant__ KArgs a) {
   using A = AR<IN, WIRE, OUT>;
-  const float pre = (a.flags & TOK_FLAG_SCALE_POST) ? 1.f : a.scale;
-  const float post = (a.flags & TOK_FLAG_SCALE_POST) ? a.scale : 1.f;
   const typename A::RI* in = static_cast<const typename A::RI*>(a.in);
   const size_t full = a.count / A::P;
-  constexpr int U = 8;
-  auto finish = [&](size_t idx, typename A::RW w) {
-    if (post != 1.f) {
-      float v[A::P];
-      A::CW::to_f32(w, v);
-#pragma unroll
-      for (int k = 0; k < A::P; ++k) v[k] *= post;
-      w = A::CW::from_f32(v);
-    }
-    A::wire_to_out(a, idx, w);
+  const Slab sl = cta_slab(a, full);
+  auto finish = [&](size_t i, const typename A::RW& w) {
+    A::wire_to_out(a, i, A::scale_wire(w, sl.post));
   };
-  const size_t lo = static_cast<size_t>(blockIdx.x) * a.packs_per_cta;
-  const size_t hi = min_sz(lo + a.packs_per_cta, full);
-  size_t i = lo + threadIdx.x;
-  for (; i + (U - 1) * kThreads < hi; i += U * kThreads) {
-    typename A::RI r[U];
-#pragma unroll
-    for (int u = 0; u < U; ++u) r[u] = __ldcs(in + i + u * kThreads);
-#pragma unroll
-    for (int u = 0; u < U; ++u) finish(i + u * kThreads, A::in_to_wire(r[u], pre));
-  }
-  for (; i < hi; i += kThreads) finish(i, A::in_to_wire(__ldcs(in + i), pre));
+  stream<8>(sl.lo, sl.hi, [&](size_t i) { return __ldcs(in + i); },
+            [&](size_t i, const typename A::RI& r) { finish(i, A::in_to_wire(r, sl.pre)); });
   if (blockIdx.x == 0 && threadIdx.x == 0 && full < a.total_packs)
-    finish(full, A::in_tail_to_wire(a, full, pre));
+    finish(full, A::in_tail_to_wire(a, full, sl.pre));
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -815,11 +819,10 @@ __global__ void __launch_bounds__(kTmaThreads) local_tma_kernel(const __grid_con
   using A = AR<T, T, T>;
   extern __shared__ __align__(128) unsigned char tma_smem[];
   uint64_t* full_bar = reinterpret_cast<uint64_t*>(tma_smem + kTmaStages * kTmaTileBytes);
-  const float pre = (a.flags & TOK_FLAG_SCALE_POST) ? 1.f : a.scale;
-  const float post = (a.flags & TOK_FLAG_SCALE_POST) ? a.scale : 1.f;
   const char* in = static_cast<const char*>(a.in);
   char* out = static_cast<char*>(a.out);
   const size_t full = a.count / A::P;
+  const Slab sl = cta_slab(a, full);  // only the scales: the tiles are strided over the grid
   const size_t nbytes = full * 16;
   const size_t ntiles = (nbytes + kTmaTileBytes - 1) / kTmaTileBytes;
   const size_t nk = ntiles > blockIdx.x ? (ntiles - blockIdx.x - 1) / gridDim.x + 1 : 0;
@@ -846,17 +849,8 @@ __global__ void __launch_bounds__(kTmaThreads) local_tma_kernel(const __grid_con
     mbar_wait(&full_bar[s], static_cast<uint32_t>((k / kTmaStages) & 1));
     typename A::RW* tile = reinterpret_cast<typename A::RW*>(tma_smem + s * kTmaTileBytes);
     const uint32_t packs = tile_len(k) / 16;
-    for (uint32_t i = tid; i < packs; i += kTmaThreads) {
-      typename A::RW w = A::in_to_wire(tile[i], pre);
-      if (post != 1.f) {
-        float v[A::P];
-        A::CW::to_f32(w, v);
-#pragma unroll
-        for (int q = 0; q < A::P; ++q) v[q] *= post;
-        w = A::CW::from_f32(v);
-      }
-      tile[i] = w;
-    }
+    for (uint32_t i = tid; i < packs; i += kTmaThreads)
+      tile[i] = A::scale_wire(A::in_to_wire(tile[i], sl.pre), sl.post);
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // generic writes -> async proxy
     __syncthreads();
     if (tid == 0) {
@@ -869,46 +863,32 @@ __global__ void __launch_bounds__(kTmaThreads) local_tma_kernel(const __grid_con
     }
   }
   if (tid == 0) bulk_wait_read<0>();  // shared memory must outlive the stores that read it
-  if (blockIdx.x == 0 && tid == 0 && full < a.total_packs) {
-    typename A::RW w = A::in_tail_to_wire(a, full, pre);
-    if (post != 1.f) {
-      float v[A::P];
-      A::CW::to_f32(w, v);
-#pragma unroll
-      for (int q = 0; q < A::P; ++q) v[q] *= post;
-      w = A::CW::from_f32(v);
-    }
-    A::wire_to_out(a, full, w);
-  }
+  if (blockIdx.x == 0 && tid == 0 && full < a.total_packs)
+    A::wire_to_out(a, full, A::scale_wire(A::in_tail_to_wire(a, full, sl.pre), sl.post));
 }
 
 template <class IN, class WIRE, class OUT>
 __global__ void __launch_bounds__(kThreads, 1) one_shot_kernel(const __grid_constant__ KArgs a) {
   using A = AR<IN, WIRE, OUT>;
-  __shared__ uint32_t s_words[3];
-  __shared__ int s_fail;
-  CtaState st = cta_begin(a, s_words, &s_fail);
+  __shared__ CtaShared sh;
+  CtaState st = cta_begin(a, sh);
+  const Slab sl = cta_slab(a, a.total_packs);
   const int q = st.seq & 1;
-  const float pre = (a.flags & TOK_FLAG_SCALE_POST) ? 1.f : a.scale;
-  const float post = (a.flags & TOK_FLAG_SCALE_POST) ? a.scale : 1.f;
-  const size_t lo = static_cast<size_t>(blockIdx.x) * a.packs_per_cta;
-  const size_t hi = min_sz(lo + a.packs_per_cta, a.total_packs);
 
   dbg_stamp(a, 0);
-  A::stage_push(a, q, lo, hi, pre);
+  A::stage_push(a, q, sl.lo, sl.hi, sl.pre);
   dbg_stamp(a, 1);
-  st.bar += 1;
-  if (cta_barrier(a, st.bar, &s_fail)) {
+  if (cta_barrier(a, st)) {
     dbg_stamp(a, 2);
     const typename A::RW* src[kMaxWorld];
 #pragma unroll
     for (int p = 0; p < kMaxWorld; ++p)
       src[p] = reinterpret_cast<const typename A::RW*>(a.peer[a.rank] + a.stage_off[q] +
                                                        static_cast<size_t>(p) * a.slot_bytes);
-    A::reduce_dispatch(a, src, nullptr, lo, hi, post);
+    A::reduce_dispatch(a, src, nullptr, sl.lo, sl.hi, sl.post);
     dbg_stamp(a, 3);
   } else {
-    A::poison(a, lo, hi);
+    A::poison(a, sl.lo, sl.hi);
   }
   cta_end(a, st);
 }
@@ -916,79 +896,55 @@ __global__ void __launch_bounds__(kThreads, 1) one_shot_kernel(const __grid_cons
 template <class IN, class WIRE, class OUT>
 __global__ void __launch_bounds__(kThreads, 1) two_shot_kernel(const __grid_constant__ KArgs a) {
   using A = AR<IN, WIRE, OUT>;
-  __shared__ uint32_t s_words[3];
-  __shared__ int s_fail;
-  CtaState st = cta_begin(a, s_words, &s_fail);
+  __shared__ CtaShared sh;
+  CtaState st = cta_begin(a, sh);
+  const Slab sl = cta_slab(a, a.total_packs);
   const int q = st.seq & 1;
-  const float pre = (a.flags & TOK_FLAG_SCALE_POST) ? 1.f : a.scale;
-  const float post = (a.flags & TOK_FLAG_SCALE_POST) ? a.scale : 1.f;
-  const size_t lo = static_cast<size_t>(blockIdx.x) * a.packs_per_cta;
-  const size_t hi = min_sz(lo + a.packs_per_cta, a.total_packs);
-  const size_t M = a.packs_per_cta / a.world;  // sub-slab length
   typename A::RW* mine = reinterpret_cast<typename A::RW*>(a.peer[a.rank] + a.stage_off[q]);
 
   dbg_stamp(a, 0);
-  A::stage_local(a, mine, lo, hi, pre);
+  A::stage_local(a, mine, sl.lo, sl.hi, sl.pre);
   dbg_stamp(a, 1);
-  st.bar += 1;
-  bool ok = cta_barrier(a, st.bar, &s_fail);
+  bool ok = cta_barrier(a, st);
   dbg_stamp(a, 2);
   if (ok) {
     const typename A::RW* src[kMaxWorld];
 #pragma unroll
     for (int p = 0; p < kMaxWorld; ++p)
       src[p] = reinterpret_cast<const typename A::RW*>(a.peer[p < a.world ? p : 0] + a.stage_off[q]);
-    const size_t slo = min_sz(lo + static_cast<size_t>(a.rank) * M, hi);
-    const size_t shi = min_sz(slo + M, hi);
-    A::reduce_dispatch(a, src, mine, slo, shi, post);
+    const Range sub = sl.sub(a.rank);
+    A::reduce_dispatch(a, src, mine, sub.lo, sub.hi, sl.post);
     dbg_stamp(a, 3);
-    st.bar += 1;
-    ok = cta_barrier(a, st.bar, &s_fail);
+    ok = cta_barrier(a, st);
     dbg_stamp(a, 4);
   }
-  if (ok)
-    A::gather_packs(a, a.stage_off[q], lo, M);
-  else
-    A::poison(a, lo, hi);
-  dbg_stamp(a, 5);
-  cta_end(a, st);
+  if (ok) A::gather_packs(a, a.stage_off[q], sl.lo, sl.M);
+  A::finish(a, st, sl, ok);
 }
 
 template <class IN, class WIRE, class OUT>
 __global__ void __launch_bounds__(kThreads, 1) nvls_kernel(const __grid_constant__ KArgs a) {
   using A = AR<IN, WIRE, OUT>;
-  __shared__ uint32_t s_words[3];
-  __shared__ int s_fail;
-  CtaState st = cta_begin(a, s_words, &s_fail);
+  __shared__ CtaShared sh;
+  CtaState st = cta_begin(a, sh);
+  const Slab sl = cta_slab(a, a.total_packs);
   const int q = st.seq & 1;
-  const float pre = (a.flags & TOK_FLAG_SCALE_POST) ? 1.f : a.scale;
-  const float post = (a.flags & TOK_FLAG_SCALE_POST) ? a.scale : 1.f;
-  const size_t lo = static_cast<size_t>(blockIdx.x) * a.packs_per_cta;
-  const size_t hi = min_sz(lo + a.packs_per_cta, a.total_packs);
-  const size_t M = a.packs_per_cta / a.world;
   typename A::RW* mine = reinterpret_cast<typename A::RW*>(a.peer[a.rank] + a.stage_off[q]);
 
   dbg_stamp(a, 0);
-  A::stage_local(a, mine, lo, hi, pre);
+  A::stage_local(a, mine, sl.lo, sl.hi, sl.pre);
   dbg_stamp(a, 1);
-  st.bar += 1;
-  bool ok = cta_barrier(a, st.bar, &s_fail);
+  bool ok = cta_barrier(a, st);
   dbg_stamp(a, 2);
   if (ok) {
-    const size_t slo = min_sz(lo + static_cast<size_t>(a.rank) * M, hi);
-    const size_t shi = min_sz(slo + M, hi);
-    A::nvls_reduce(a, a.mc + a.stage_off[q], slo, shi, post);
+    const Range sub = sl.sub(a.rank);
+    A::nvls_reduce(a, a.mc + a.stage_off[q], sub.lo, sub.hi, sl.post);
     dbg_stamp(a, 3);
-    st.bar += 1;
-    ok = cta_barrier(a, st.bar, &s_fail);
+    ok = cta_barrier(a, st);
     dbg_stamp(a, 4);
   }
-  if (ok)
-    A::copy_out(a, mine, lo, hi);
-  else
-    A::poison(a, lo, hi);
-  dbg_stamp(a, 5);
-  cta_end(a, st);
+  if (ok) A::copy_out(a, mine, sl.lo, sl.hi);
+  A::finish(a, st, sl, ok);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1043,65 +999,49 @@ __global__ void __launch_bounds__(32) arrive_kernel(const __grid_constant__ KArg
 template <class WIRE>
 __global__ void __launch_bounds__(kThreads, 1) nvls_inplace_kernel(const __grid_constant__ KArgs a) {
   using A = AR<WIRE, WIRE, WIRE>;
-  __shared__ uint32_t s_words[3];
-  __shared__ int s_fail;
-  CtaState st = cta_begin(a, s_words, &s_fail);
-  const size_t lo = static_cast<size_t>(blockIdx.x) * a.packs_per_cta;
-  const size_t hi = min_sz(lo + a.packs_per_cta, a.total_packs);
-  const size_t M = a.packs_per_cta / a.world;
+  __shared__ CtaShared sh;
+  CtaState st = cta_begin(a, sh);
+  const Slab sl = cta_slab(a, a.total_packs);
   dbg_stamp(a, 0);
   bool ok = st.arrived == 0;
   dbg_stamp(a, 2);
   if (ok) {
-    const size_t slo = min_sz(lo + static_cast<size_t>(a.rank) * M, hi);
-    const size_t shi = min_sz(slo + M, hi);
-    if (a.unroll == 16)                                       // the switch sums; scale the sum
-      A::template nvls_reduce<16>(a, a.mc + a.buf_off, slo, shi, a.scale);
+    const Range sub = sl.sub(a.rank);
+    if (a.unroll == 16)  // the switch sums; scale the sum
+      A::template nvls_reduce<16>(a, a.mc + a.buf_off, sub.lo, sub.hi, a.scale);
     else
-      A::template nvls_reduce<8>(a, a.mc + a.buf_off, slo, shi, a.scale);
+      A::template nvls_reduce<8>(a, a.mc + a.buf_off, sub.lo, sub.hi, a.scale);
     dbg_stamp(a, 3);
-    st.bar += 1;
-    ok = cta_barrier<false>(a, st.bar, &s_fail);
+    ok = cta_barrier<false>(a, st);
     dbg_stamp(a, 4);
   }
-  if (!ok) A::poison(a, lo, hi);
-  dbg_stamp(a, 5);
-  cta_end(a, st);
+  A::finish(a, st, sl, ok);
 }
 
 template <class WIRE>
 __global__ void __launch_bounds__(kThreads, 1)
     two_shot_inplace_kernel(const __grid_constant__ KArgs a) {
   using A = AR<WIRE, WIRE, WIRE>;
-  __shared__ uint32_t s_words[3];
-  __shared__ int s_fail;
-  CtaState st = cta_begin(a, s_words, &s_fail);
-  const float pre = (a.flags & TOK_FLAG_SCALE_POST) ? 1.f : a.scale;
-  const float post = (a.flags & TOK_FLAG_SCALE_POST) ? a.scale : 1.f;
-  const size_t lo = static_cast<size_t>(blockIdx.x) * a.packs_per_cta;
-  const size_t hi = min_sz(lo + a.packs_per_cta, a.total_packs);
-  const size_t M = a.packs_per_cta / a.world;
+  __shared__ CtaShared sh;
+  CtaState st = cta_begin(a, sh);
+  const Slab sl = cta_slab(a, a.total_packs);
   dbg_stamp(a, 0);
   bool ok = st.arrived == 0;
   dbg_stamp(a, 2);
   if (ok) {
-    const size_t slo = min_sz(lo + static_cast<size_t>(a.rank) * M, hi);
-    const size_t shi = min_sz(slo + M, hi);
+    const Range sub = sl.sub(a.rank);
     // reduce-scatter (reads over NVLink) fused with a push all-gather (posted writes over NVLink)
     if (a.world <= 2)
-      A::template reduce_push<2, 8>(a, slo, shi, pre, post);
+      A::template reduce_push<2, 8>(a, sub.lo, sub.hi, sl.pre, sl.post);
     else if (a.world <= 4)
-      A::template reduce_push<4, 4>(a, slo, shi, pre, post);
+      A::template reduce_push<4, 4>(a, sub.lo, sub.hi, sl.pre, sl.post);
     else
-      A::template reduce_push<kMaxWorld, 2>(a, slo, shi, pre, post);
+      A::template reduce_push<kMaxWorld, 2>(a, sub.lo, sub.hi, sl.pre, sl.post);
     dbg_stamp(a, 3);
-    st.bar += 1;
-    ok = cta_barrier<false>(a, st.bar, &s_fail);
+    ok = cta_barrier<false>(a, st);
     dbg_stamp(a, 4);
   }
-  if (!ok) A::poison(a, lo, hi);
-  dbg_stamp(a, 5);
-  cta_end(a, st);
+  A::finish(a, st, sl, ok);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1116,15 +1056,13 @@ __global__ void __launch_bounds__(kThreads, 1)
 // ------------------------------------------------------------------------------------------------
 template <int MODE>
 __global__ void __launch_bounds__(kThreads, 1) bcast_kernel(const __grid_constant__ KArgs a) {
-  __shared__ uint32_t s_words[3];
-  __shared__ int s_fail;
-  CtaState st = cta_begin(a, s_words, &s_fail);
+  __shared__ CtaShared sh;
+  CtaState st = cta_begin(a, sh);
   const int q = st.seq & 1;
   const size_t packs = a.count / 16;  // whole 16-byte packs; the byte tail is handled below
   const size_t lo = min_sz(static_cast<size_t>(blockIdx.x) * a.packs_per_cta, packs);
   const size_t hi = min_sz(lo + a.packs_per_cta, packs);
   const bool root = a.rank == a.root;
-  constexpr int U = 8;
   bool ok = true;
   if (MODE == kBcastStaged) {
     uint4* stage = reinterpret_cast<uint4*>(a.peer[a.root] + a.stage_off[q]);
@@ -1135,19 +1073,11 @@ __global__ void __launch_bounds__(kThreads, 1) bcast_kernel(const __grid_constan
         reinterpret_cast<char*>(stage)[packs * 16 + threadIdx.x] =
             static_cast<const char*>(a.in)[packs * 16 + threadIdx.x];
     }
-    st.bar += 1;
-    ok = cta_barrier(a, st.bar, &s_fail);
+    ok = cta_barrier(a, st);
     if (ok && !root) {
       uint4* dst = static_cast<uint4*>(a.out);
-      size_t i = lo + threadIdx.x;
-      for (; i + (U - 1) * kThreads < hi; i += U * kThreads) {
-        uint4 r[U];
-#pragma unroll
-        for (int u = 0; u < U; ++u) r[u] = ld_sys(stage + i + u * kThreads);
-#pragma unroll
-        for (int u = 0; u < U; ++u) dst[i + u * kThreads] = r[u];
-      }
-      for (; i < hi; i += kThreads) dst[i] = ld_sys(stage + i);
+      stream<8>(lo, hi, [&](size_t i) { return ld_sys(stage + i); },
+                [&](size_t i, const uint4& v) { dst[i] = v; });
       if (blockIdx.x == 0 && threadIdx.x < (a.count & 15)) {
         const volatile char* sb = reinterpret_cast<const volatile char*>(stage);
         static_cast<char*>(a.out)[packs * 16 + threadIdx.x] = sb[packs * 16 + threadIdx.x];
@@ -1160,6 +1090,8 @@ __global__ void __launch_bounds__(kThreads, 1) bcast_kernel(const __grid_constan
         if (root) {
           const uint4* src = reinterpret_cast<const uint4*>(a.peer[a.rank] + a.buf_off);
           uint4* mc = reinterpret_cast<uint4*>(a.mc + a.buf_off);
+          // written out: on stream() this loop compiles to differently scheduled machine code
+          constexpr int U = 8;
           size_t i = lo + threadIdx.x;
           for (; i + (U - 1) * kThreads < hi; i += U * kThreads) {
             uint4 r[U];
@@ -1173,18 +1105,10 @@ __global__ void __launch_bounds__(kThreads, 1) bcast_kernel(const __grid_constan
       } else if (!root) {
         const uint4* src = reinterpret_cast<const uint4*>(a.peer[a.root] + a.buf_off);
         uint4* dst = reinterpret_cast<uint4*>(a.peer[a.rank] + a.buf_off);
-        size_t i = lo + threadIdx.x;
-        for (; i + (U - 1) * kThreads < hi; i += U * kThreads) {
-          uint4 r[U];
-#pragma unroll
-          for (int u = 0; u < U; ++u) r[u] = ld_sys(src + i + u * kThreads);
-#pragma unroll
-          for (int u = 0; u < U; ++u) dst[i + u * kThreads] = r[u];
-        }
-        for (; i < hi; i += kThreads) dst[i] = ld_sys(src + i);
+        stream<8>(lo, hi, [&](size_t i) { return ld_sys(src + i); },
+                  [&](size_t i, const uint4& v) { dst[i] = v; });
       }
-      st.bar += 1;
-      ok = cta_barrier(a, st.bar, &s_fail);
+      ok = cta_barrier(a, st);
     }
   }
   cta_end(a, st);
@@ -1192,7 +1116,8 @@ __global__ void __launch_bounds__(kThreads, 1) bcast_kernel(const __grid_constan
 
 // ------------------------------------------------------------------------------------------------
 // Profiling aid (tools/barrier_bench.py): `count` cross-replica barriers back to back, nothing else —
-// what one barrier costs, and which part of it.  Variants:
+// what one barrier costs, and which part of it.  Every variant runs warp_barrier, the routine of the
+// exchange kernels' cta_barrier:
 //   0 production barrier (multimem.red.release when a multicast mapping exists, else P2P flags)
 //   1 production P2P-flag barrier even when a multicast mapping exists
 //   2 signalling only: relaxed multimem.red + relaxed poll, no release, no acquire fence
@@ -1205,7 +1130,8 @@ __global__ void __launch_bounds__(kThreads, 1) barrier_bench_kernel(const __grid
   const int variant = static_cast<int>(a.flags);
   // the multicast counters (slots 192..255) and the P2P flags (slots 128..191) count separately
   const bool mc_variant = a.mc != nullptr && (variant == 0 || variant == 2 || variant == 4);
-  const int slot = (mc_variant ? 192 : 128) + blockIdx.x;
+  const bool ordered = variant == 0 || variant == 1 || variant == 4;
+  const uint32_t slot = (mc_variant ? 192 : 128) + blockIdx.x;
   if (threadIdx.x == 0) s_fail = 0;
   uint32_t bar = a.ctr[slot];
   __syncthreads();
@@ -1219,44 +1145,7 @@ __global__ void __launch_bounds__(kThreads, 1) barrier_bench_kernel(const __grid
       for (int k = 0; k < 8; ++k) dst[threadIdx.x + k * kThreads] = v;
     }
     __syncthreads();
-    if (threadIdx.x < 32) {
-      const int lane = threadIdx.x;
-      const bool use_mc = a.mc != nullptr && (variant == 0 || variant == 2 || variant == 4);
-      const bool ordered = variant == 0 || variant == 1 || variant == 4;
-      const uint32_t* word;
-      uint32_t want;
-      bool polls;
-      if (use_mc) {
-        uint32_t* mcw = reinterpret_cast<uint32_t*>(a.mc + kMcntOff) + slot;
-        if (lane == 0) {
-          if (ordered)
-            multimem_red_release_add(mcw, 1u);
-          else
-            asm volatile("multimem.red.relaxed.sys.global.add.u32 [%0], %1;" ::"l"(mcw), "r"(1u)
-                         : "memory");
-        }
-        word = reinterpret_cast<const uint32_t*>(a.peer[a.rank] + kMcntOff) + slot;
-        want = bar * static_cast<uint32_t>(a.world);
-        polls = lane == 0;
-      } else {
-        polls = lane < a.world;
-        if (polls) {
-          uint32_t* dst = reinterpret_cast<uint32_t*>(a.peer[lane]) + (slot * kMaxWorld + a.rank);
-          if (ordered)
-            st_release_sys(dst, bar);
-          else
-            asm volatile("st.relaxed.sys.global.u32 [%0], %1;" ::"l"(dst), "r"(bar) : "memory");
-        }
-        word = reinterpret_cast<const uint32_t*>(a.peer[a.rank]) + (slot * kMaxWorld + (polls ? lane : 0));
-        want = bar;
-      }
-      const int code = warp_spin(a, word, want, polls, 3u);
-      if (code != 0 && lane == 0) {
-        a.hostctl[kCtlStatus] = code;
-        s_fail = 1;
-      }
-      if (ordered) fence_sys();
-    }
+    if (threadIdx.x < 32) warp_barrier(a, slot, bar, mc_variant, ordered, ordered, &s_fail);
     __syncthreads();
     if (s_fail) break;
   }
